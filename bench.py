@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RAG /retrieve queries/sec on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[2] "hybrid dense+BM25+RRF /retrieve, 10M docs
@@ -17,6 +17,10 @@ One JSON line on rank 0:
   roofline: dominant kernel (dense scan) algorithmic GB/s against MEASURED_PEAKS.json
   cpu_baseline / --impl reference: the CPU oracle (restated reference path; faiss/bm25s are not
             installable offline) on all host cores over a bounded sample, extrapolated linearly in N.
+
+--dump-outputs DIR writes the /retrieve result of the last timed step of `value` as DIR/<name>.npy (float32 / float64;
+integer outputs as exact float64; a missing score, NaN in the result, as 0 with <name>_present.npy = 0 beside it).  The
+inputs depend only on the arguments, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -100,7 +104,38 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-optin", action="store_true", help="skip the extra OPT-IN measurement (bf16 shadow prune pass) after the default one")
     ap.add_argument("--cpu-sample-rows", type=int, default=40_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step returned to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> [B, ...] results of one step.  The fuse kernel marks a score that does not exist (a candidate only
+    one list found, a slot past count) with NaN: every float array is stored with those entries as 0 and a 0/1 mask
+    <name>_present.npy, so all files are finite.  Integer arrays are stored as float64 (exact below 2^53).  Above
+    DUMP_LIMIT bytes in all, a fixed seeded sample of the B rows is stored, with its row indices as rows.npy."""
+    out = {}
+    for n, a in arrays.items():
+        if a.dtype.kind == "f":
+            ok = np.isfinite(a)
+            out[n], out[n + "_present"] = np.where(ok, a, 0).astype(a.dtype), ok.astype(np.float32)
+        else:
+            out[n] = a.astype(np.float64)
+    arrays = out
+    B = len(next(iter(arrays.values())))
+    per_row = sum(a.nbytes for a in arrays.values()) / B
+    if per_row * B > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(B, int((DUMP_LIMIT - 65536) // (per_row + 8)), replace=False))   # .npy headers
+        arrays = {n: a[rows] for n, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
 
 
 # ------------------------------------------------------------------------- helpers
@@ -476,6 +511,8 @@ def run_ours(args):
             return sr.retrieve(None, terms_list, k, embedder=embedder, tokens=(flat_tok, tok_off))
         return sr.retrieve(qh, terms_list, k)
 
+    last = {}
+
     def timed(fn, steps, warmup):
         for _ in range(warmup):
             fn()
@@ -483,7 +520,7 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last["out"] = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
@@ -497,6 +534,8 @@ def run_ours(args):
     l0 = ctx.launch_count()
     trace("timed ms_dev")
     ms_dev = timed(step_dev, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:          # the result buffers are reused by the legs below: copy them out now
+        dump_outputs(args.dump_outputs, {n: t.cpu().numpy() for n, t in last["out"].items()})
     launches = (ctx.launch_count() - l0) // (args.steps + args.warmup) * args.steps
     trace("timed ms_e2e")
     ms_e2e = timed(step_e2e, args.steps, args.warmup)

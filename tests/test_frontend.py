@@ -2,7 +2,10 @@
 RPC (kaito_b200/rpc.py), everything else reverse-proxied to the engine's FastAPI app.  Answers, error bodies and metrics must be
 those of the single-process service (presets/ragengine/main.py:742-771)."""
 import json
+import os
+import shutil
 import socket
+import tempfile
 import threading
 import time
 import urllib.error
@@ -21,6 +24,15 @@ def _free_port():
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         return s.getsockname()[1]
+
+
+@pytest.fixture
+def rpc_path():
+    """unix-socket path in a fresh directory under /tmp: a socket path is limited to 107 bytes, which pytest's tmp_path
+    exceeds when TMPDIR is deep"""
+    d = tempfile.mkdtemp(prefix="krag-", dir="/tmp")
+    yield os.path.join(d, "rpc.sock")
+    shutil.rmtree(d, ignore_errors=True)
 
 
 def _http(method, url, body=None):
@@ -42,7 +54,7 @@ def test_parse_retrieve_matches_the_request_model():
         assert ok(bad, 300) is None, bad
 
 
-def test_worker_process_serves_retrieve_and_proxies_the_rest(oracle, tmp_path):
+def test_worker_process_serves_retrieve_and_proxies_the_rest(oracle, tmp_path, rpc_path):
     import uvicorn
     from fastapi import HTTPException as FHE
     from tests.oracle_engine import OracleEngine
@@ -54,7 +66,7 @@ def test_worker_process_serves_retrieve_and_proxies_the_rest(oracle, tmp_path):
     th.start()
     while not srv.started:
         time.sleep(0.02)
-    rpc = RetrieveRpcServer(app.state.batcher, app.state.observe_retrieve, (vs.HTTPException, FHE), path=str(tmp_path / "rpc.sock"))
+    rpc = RetrieveRpcServer(app.state.batcher, app.state.observe_retrieve, (vs.HTTPException, FHE), path=rpc_path)
     procs = frontend.spawn(1, "127.0.0.1", public_port, f"127.0.0.1:{engine_port}", rpc.path, None, RAG_MAX_TOP_K)
     base = f"http://127.0.0.1:{public_port}"
     try:
@@ -109,7 +121,7 @@ def test_worker_process_serves_retrieve_and_proxies_the_rest(oracle, tmp_path):
         app.state.batcher.close()
 
 
-def test_rpc_client_survives_an_engine_restart(oracle, tmp_path):
+def test_rpc_client_survives_an_engine_restart(oracle, rpc_path):
     """the worker's connection to the engine is re-established on the next request after it broke; requests in flight at the
     time fail with ConnectionError (the worker answers 503)"""
     import asyncio
@@ -120,15 +132,14 @@ def test_rpc_client_survives_an_engine_restart(oracle, tmp_path):
     store = VectorStore(HashingEmbedding(64), OracleEngine(oracle))
     store.index_documents("r", [{"text": f"alpha beta {i}"} for i in range(12)])
     seen = []
-    path = str(tmp_path / "rpc.sock")
 
     def start():
         b = RetrieveBatcher(store, max_batch=16, max_wait_s=0.002)
-        return b, RetrieveRpcServer(b, lambda status, seconds, out: seen.append(status), (vs.HTTPException, FHE), path=path)
+        return b, RetrieveRpcServer(b, lambda status, seconds, out: seen.append(status), (vs.HTTPException, FHE), path=rpc_path)
 
     async def scenario():
         b, srv = start()
-        cli = RetrieveRpcClient(path)
+        cli = RetrieveRpcClient(rpc_path)
         st, body = await cli.retrieve("r", "alpha 3", 2, None)
         assert st == 200 and json.loads(body)["count"] == 2
         st, body = await cli.retrieve("nope", "q", 2, None)

@@ -9,8 +9,8 @@ import re
 import socket
 import threading
 import time
-
-import pytest
+import urllib.request
+from datetime import datetime
 
 from kaito_b200.embedding import HashingEmbedding
 from kaito_b200.service import create_app, resolve_model_dir
@@ -102,45 +102,58 @@ def test_prestop_snapshot_and_poststart_restore(oracle, tmp_path, monkeypatch):
         th.join(timeout=5)
 
 
-REF_MANAGER = "/root/reference/presets/ragengine/lifecycle/manager.py"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lifecycle_reference.json")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_MANAGER), reason="reference tree not present (it never is on the GPU box)")
+def _replay(url, requests, snapshot):
+    """send recorded requests (URLs as the reference's hooks sent them) and check each answer against the recording"""
+    for r in requests:
+        req = urllib.request.Request(url + r["url"].replace("{snapshot}", snapshot), method=r["method"],
+                                     data=b"" if r["method"] == "POST" else None)
+        with urllib.request.urlopen(req, timeout=30) as resp:
+            assert (resp.status, json.loads(resp.read())) == (r["status"], json.loads(json.dumps(r["body"]).replace("{snapshot}", snapshot)))
+
+
 def test_reference_lifecycle_manager_drives_this_service(oracle, tmp_path, monkeypatch):
-    """Drop-in check with the reference in the loop: its own PreStop/PostStart handlers (lifecycle/manager.py, executed
-    unmodified, only pointed at the test server) persist and restore this service's indexes, and snapshots written by
-    either implementation restore under the other."""
+    """Drop-in check against the reference's own PreStop/PostStart handlers (lifecycle/manager.py), replayed from
+    tests/golden/lifecycle_reference.json (oracle/gen_golden_lifecycle.py ran them against this service): a snapshot laid
+    out by the reference's PreStop restores under our PostStart, and the reference's PostStart requests restore a snapshot
+    written by our PreStop."""
     from starlette.testclient import TestClient
     from tests.oracle_engine import OracleEngine
+    gold = json.load(open(GOLD))
+    pre = gold["prestop"]
     port = _free_port()
     url = f"http://127.0.0.1:{port}"
     app = create_app(VectorStore(HashingEmbedding(64), OracleEngine(oracle)), {"persist_dir": str(tmp_path), "llm_inference_url": None})
     server, th = _serve(app, port)
     try:
-        spec = importlib.util.spec_from_file_location("ref_lifecycle_manager", REF_MANAGER)
-        ref = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref)
-        ref.wait_for_service.__defaults__ = (url + "/indexes", 60)
-        for fn in (ref.get_indexes, ref.load_index, ref.persist_index):
-            fn.__defaults__ = (url,)
-        import types
-        monkeypatch.setattr(ref, "time", types.SimpleNamespace(sleep=lambda s: None, time=time.time))   # its 0.5 s rate limiting
-        monkeypatch.setenv("POD_UID", "feedfacecafe")
+        monkeypatch.setenv("POD_UID", gold["pod_uid"])
         c = TestClient(app)
-        docs = [{"text": "First document about retrieval engines"}, {"text": "Second document about Kubernetes operators"}]
-        assert c.post("/index", json={"index_name": "idx_a", "documents": docs}).status_code == 200
+        assert c.post("/index", json={"index_name": "idx_a", "documents": gold["documents"]}).status_code == 200
         before = c.post("/retrieve", json={"index_name": "idx_a", "query": "retrieval engines", "max_node_count": 2}).json()
         # reference PreStop -> our PostStart
-        assert ref.prestop_handler(str(tmp_path)) == 0
+        name = pre["snapshot_name"].replace("{timestamp}", datetime.now().strftime(pre["snapshot_timestamp_format"]))
+        snap = tmp_path / "systemsnapshots" / name
+        snap.mkdir(parents=True)
+        _replay(url, pre["requests"], str(snap))
+        meta = dict(pre["metadata"], timestamp=datetime.now().isoformat())
+        (snap / "metadata.json").write_text(json.dumps(meta, indent=2))
+        os.symlink(pre["latest"].replace("{snapshot_name}", name), tmp_path / "LATEST")
         assert c.delete("/indexes/idx_a").status_code == 200
-        hooks = _load_hooks(monkeypatch, port, tmp_path, "feedfacecafe")
+        hooks = _load_hooks(monkeypatch, port, tmp_path, gold["pod_uid"])
         assert hooks.poststart() == 0
         assert c.post("/retrieve", json={"index_name": "idx_a", "query": "retrieval engines", "max_node_count": 2}).json() == before
-        # our PreStop -> reference PostStart
+        # our PreStop -> reference PostStart: the layout its handler reads, then the requests it sends
         time.sleep(1.1)
         assert hooks.prestop() == 0
+        latest = os.readlink(tmp_path / "LATEST")
+        assert re.fullmatch(re.escape(pre["latest"]).replace(re.escape("{snapshot_name}"), r"\d{4}-\d\d-\d\dT\d\d-\d\d-\d\d_pod-")
+                            + re.escape(pre["metadata"]["pod_uid"]), latest)
+        ours = json.load(open(tmp_path / latest / "metadata.json"))
+        assert set(ours) == set(pre["metadata"]) and ours["index_names"] == pre["metadata"]["index_names"]
         assert c.delete("/indexes/idx_a").status_code == 200
-        assert ref.poststart_handler(str(tmp_path)) == 0
+        _replay(url, gold["poststart"]["requests"], os.path.realpath(tmp_path / "LATEST"))
         assert c.get("/indexes").json() == ["idx_a"]
         assert c.post("/retrieve", json={"index_name": "idx_a", "query": "retrieval engines", "max_node_count": 2}).json() == before
         assert len(os.listdir(tmp_path / "systemsnapshots")) == 2
@@ -183,30 +196,26 @@ def test_resolve_model_dir(tmp_path, monkeypatch):
     assert resolve_model_dir("BAAI/bge-small-en-v1.5") == str(tmp_path / "explicit")
 
 
-REF_GO = "/root/reference/pkg/ragengine"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_GO), reason="reference tree not present")
 def test_deploy_tree_satisfies_the_controllers_pod_contract():
     """The literals the unmodified controller puts into the pod spec (pkg/ragengine/manifests/manifests.go:116-134, 146-279;
-    pkg/ragengine/controllers/preset_rag.go:33-64, 186) resolve inside deploy/: hook script path and verbs, `python3 main.py` in
-    the image WORKDIR, port and probe path, and the environment variables the hooks read."""
+    pkg/ragengine/controllers/preset_rag.go:33-64, 186), stored in tests/golden/lifecycle_reference.json, resolve inside
+    deploy/: hook script path and verbs, `python3 main.py` in the image WORKDIR, port and probe path, and the environment
+    variables the hooks read."""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    man = open(os.path.join(REF_GO, "manifests", "manifests.go")).read()
-    pre = open(os.path.join(REF_GO, "controllers", "preset_rag.go")).read()
-    hook_path = re.search(r'"(/app/ragengine/lifecycle/hooks\.py)"', man).group(1)
+    pod = json.load(open(GOLD))["pod_contract"]
+    assert pod["poststart_command"] == ["python3", "/app/ragengine/lifecycle/hooks.py", "poststart"]
+    hook_path = pod["poststart_command"][1]
     assert os.path.isfile(os.path.join(root, "deploy", hook_path.lstrip("/")))
-    assert "python3 /app/ragengine/lifecycle/hooks.py prestop" in man and '"poststart"' in man
+    assert f"python3 {hook_path} prestop" in pod["prestop_command"][-1]
     hooks_src = open(os.path.join(root, "deploy", hook_path.lstrip("/"))).read()
     for verb in ("poststart", "prestop"):
         assert f'"{verb}"' in hooks_src
-    for env in ("POD_NAME", "POD_UID", "DEFAULT_VECTOR_DB_PERSIST_DIR"):
-        assert f'Name:  "{env}"' in man or f'Name: "{env}"' in man
+    assert pod["env"] == ["POD_NAME", "POD_UID", "DEFAULT_VECTOR_DB_PERSIST_DIR"]
+    for env in pod["env"]:
         assert env in hooks_src
-    assert 'utils.ShellCmd("python3 main.py")' in pre and os.path.isfile(os.path.join(root, "deploy", "app", "ragengine", "main.py"))
+    assert pod["container_command"] == "python3 main.py" and os.path.isfile(os.path.join(root, "deploy", "app", "ragengine", "main.py"))
     dockerfile = open(os.path.join(root, "deploy", "Dockerfile")).read()
     assert "WORKDIR /app/ragengine" in dockerfile and "python3 main.py" in dockerfile and "EXPOSE 5000" in dockerfile
-    port = int(re.search(r"PortInferenceServer\s*=\s*(\d+)", pre).group(1))
-    probe = re.search(r'ProbePath\s*=\s*"([^"]+)"', pre).group(1)
+    port, probe = pod["port"], pod["probe_path"]
     svc = open(os.path.join(root, "kaito_b200", "service.py")).read()
     assert f"port={port}" in svc and f'@app.get("{probe}"' in svc
