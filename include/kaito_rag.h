@@ -210,6 +210,9 @@ int32_t krag_index_read_rows(krag_index* idx, int64_t row0, int64_t n, float* ou
 /* copy the postings of one term back to host: returns count via *n_out (cap entries max) */
 int32_t krag_index_read_postings(krag_index* idx, uint32_t term, int64_t cap, uint32_t* docs_out, float* scores_out,
                                  int64_t* n_out);
+/* copy the rank-table row of one term back to host: out[i] = the 2^i-th best posting score of the term, i = 0..10
+ * (0 where the term has fewer than 2^i postings) */
+int32_t krag_index_read_rank_scores(krag_index* idx, uint32_t term, float* out /*[11]*/);
 
 /* ----------------------------------------- peer-memory candidate exchange (one process per GPU, one box) */
 /* The all-gather + merge of the per-shard candidate lists done by our own kernels over NVLink peer memory:

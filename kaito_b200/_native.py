@@ -30,7 +30,7 @@ SYMBOLS = [
     "krag_index_commit", "krag_index_commit_local", "krag_index_commit_global", "krag_index_stats",
     "krag_index_node_ids", "krag_index_set_ordinal_map", "krag_index_persist", "krag_index_load", "krag_search_dense", "krag_search_bm25",
     "krag_retrieve", "krag_dev_dense_candidates", "krag_dev_bm25_candidates", "krag_dev_merge", "krag_dev_fuse",
-    "krag_synth_fill", "krag_index_read_rows", "krag_index_read_postings", "krag_tc_fallback_queries",
+    "krag_synth_fill", "krag_index_read_rows", "krag_index_read_postings", "krag_index_read_rank_scores", "krag_tc_fallback_queries",
     "krag_debug_tc_dump", "krag_last_dense_kernel", "krag_embedder_create", "krag_embedder_load_tensor",
     "krag_embedder_finalize", "krag_embed", "krag_embed_dev", "krag_embedder_destroy", "krag_debug_gemm_tf32",
     "krag_debug_linear_ln", "krag_index_set_dense_mode", "krag_text_analyze", "krag_wordpiece_create",
@@ -105,6 +105,7 @@ def load() -> C.CDLL:
     L.krag_synth_fill.argtypes = [vp, i64, i64, C.c_uint64, i64]
     L.krag_index_read_rows.argtypes = [vp, i64, i64, vp]
     L.krag_index_read_postings.argtypes = [vp, u32, i64, vp, vp, C.POINTER(i64)]
+    L.krag_index_read_rank_scores.argtypes = [vp, u32, vp]
     L.krag_embedder_create.argtypes = [vp, C.POINTER(BertConfig), C.POINTER(vp)]
     L.krag_embedder_load_tensor.argtypes = [vp, C.c_char_p, vp, i64]
     L.krag_embedder_finalize.argtypes = [vp]
@@ -448,3 +449,9 @@ class Index:
         check(self._L.krag_index_read_postings(self._h, term, cap, ptr(docs), ptr(scores), C.byref(cnt)))
         m = min(cnt.value, cap)
         return docs[:m], scores[:m], cnt.value
+
+    def read_rank_scores(self, term: int) -> np.ndarray:
+        """rank-table row of a term: [i] = its 2^i-th best posting score (i = 0..10), 0 below df"""
+        out = np.empty(11, np.float32)
+        check(self._L.krag_index_read_rank_scores(self._h, term, ptr(out)))
+        return out

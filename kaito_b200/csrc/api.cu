@@ -171,6 +171,7 @@ struct krag_index {
     Postings post;
     DevArray<uint32_t> entry_doc;  // scratch kept between commit_local and commit_global
     bool committed = false;
+    bool removed_since_commit = false;   // the alive bitmap admits fewer documents than the postings were built from
     int64_t committed_rows = 0;
     int64_t vocab = 0, n_docs_global = 0, total_len_global = 0;
     int64_t ord_base = 0, ord_stride = 1;   // global ordinal of local row r = ord_base + r * ord_stride
@@ -244,7 +245,7 @@ void bm25_candidates_dev(krag_index* ix, Slot* s, const uint32_t* d_terms, const
     }
     s->part.reserve((int64_t)bm25_part_elems(ix->committed_rows, batch, P), 0, st);
     s->bm25_res.reserve((int64_t)bm25_resolve_bytes(ix->committed_rows, n_terms_total), 0, st);
-    launch_bm25(ix->ctx->di, ix->post, ix->committed_rows, eligible ? eligible : alive_ptr(ix), d_terms, d_toff, n_terms_total, s->bm25_res.p, batch, P,
+    launch_bm25(ix->ctx->di, ix->post, ix->committed_rows, eligible ? eligible : alive_ptr(ix), !eligible && !ix->removed_since_commit, d_terms, d_toff, n_terms_total, s->bm25_res.p, batch, P,
                 ord_map(ix), s->part.p, d_keys, st);
 }
 
@@ -365,6 +366,7 @@ void commit_global_impl(krag_index* ix, int64_t vocab, const uint32_t* df_global
     ix->total_len_global = total_len_global;
     ix->ord_base = ord_base;
     ix->committed = true;
+    ix->removed_since_commit = false;
     ix->committed_rows = ix->n_rows;
 }
 
@@ -459,6 +461,7 @@ int32_t krag_index_drop(krag_index* ix)
             if (ix->post.off) cudaFree(ix->post.off);
             if (ix->post.doc) cudaFree(ix->post.doc);
             if (ix->post.score) cudaFree(ix->post.score);
+            if (ix->post.rank_score) cudaFree(ix->post.rank_score);
             if (ix->post.tile_slot) cudaFree(ix->post.tile_slot);
             if (ix->post.tile_off) cudaFree(ix->post.tile_off);
         }
@@ -562,7 +565,7 @@ int32_t krag_index_remove(krag_index* ix, int64_t n, const uint64_t* node_ids, i
             ++removed;
         }
         KRAG_CUDA(cudaStreamSynchronize(ix->ctx->admin));
-        if (removed) { ix->has_dead = true; ix->n_live -= removed; }
+        if (removed) { ix->has_dead = true; ix->removed_since_commit = true; ix->n_live -= removed; }
         if (n_removed) *n_removed = removed;
     });
 }
@@ -871,6 +874,18 @@ int32_t krag_index_read_postings(krag_index* ix, uint32_t term, int64_t cap, uin
         int64_t m = cnt < cap ? cnt : cap;
         if (m > 0 && docs_out) KRAG_CUDA(cudaMemcpy(docs_out, ix->post.doc + be[0], sizeof(uint32_t) * (size_t)m, cudaMemcpyDeviceToHost));
         if (m > 0 && scores_out) KRAG_CUDA(cudaMemcpy(scores_out, ix->post.score + be[0], sizeof(float) * (size_t)m, cudaMemcpyDeviceToHost));
+    });
+}
+
+int32_t krag_index_read_rank_scores(krag_index* ix, uint32_t term, float* out)
+{
+    return guarded([&] {
+        KRAG_REQUIRE(ix && out, KRAG_E_INVALID, "null argument");
+        std::shared_lock<std::shared_mutex> lk(ix->mu);
+        KRAG_REQUIRE(ix->committed, KRAG_E_STATE, "index not committed");
+        KRAG_REQUIRE((int64_t)term < ix->post.vocab, KRAG_E_INVALID, "term id out of range");
+        KRAG_CUDA(cudaSetDevice(ix->ctx->di.device));
+        KRAG_CUDA(cudaMemcpy(out, ix->post.rank_score + (size_t)term * BM25_RANKS, sizeof(float) * BM25_RANKS, cudaMemcpyDeviceToHost));
     });
 }
 

@@ -177,6 +177,118 @@ __global__ void tile_index_kernel(const uint32_t* __restrict__ sorted_terms, con
         if (p == e - 1) for (int64_t tl = tile_d + 1; tl <= n_tiles; ++tl) row[tl] = (uint32_t)(e - b);
     }
 }
+
+// ---- rank table (Postings::rank_score), built per term range right after its scores.  Scores are compared as
+// f32_ordered_bits keys and written back from the same bits: the table holds stored posting scores bit for bit.
+constexpr int RK_TOP = 1 << (BM25_RANKS - 1);     // 1024: deepest rank of the table
+constexpr int RS_WARPS = 8;
+// terms with 1 <= df <= RK_TOP: one warp per term, bitonic sort (descending) of the term's keys in shared memory
+__global__ void __launch_bounds__(RS_WARPS * 32)
+rank_small_kernel(const int64_t* __restrict__ off, const float* __restrict__ score, int64_t t_lo, int64_t t_hi,
+                  float* __restrict__ rank)
+{
+    __shared__ uint32_t s_key[RS_WARPS][RK_TOP];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint32_t* key = s_key[warp];
+    for (int64_t t = t_lo + (int64_t)blockIdx.x * RS_WARPS + warp; t < t_hi; t += (int64_t)gridDim.x * RS_WARPS) {
+        const int64_t b = off[t], df = off[t + 1] - b;
+        if (df == 0 || df > RK_TOP) continue;
+        const int n = (int)df, n2 = next_pow2(max(n, 2));
+        for (int i = lane; i < n2; i += 32) key[i] = i < n ? f32_ordered_bits(score[b + i]) : 0u;   // 0: below every score
+        __syncwarp();
+        for (int k = 2; k <= n2; k <<= 1) {
+            for (int j = k >> 1; j > 0; j >>= 1) {
+                for (int p = lane; p < (n2 >> 1); p += 32) {
+                    const int i = ((p & ~(j - 1)) << 1) | (p & (j - 1)), q = i | j;
+                    const uint32_t a = key[i], c = key[q];
+                    if ((a < c) == ((i & k) == 0)) { key[i] = c; key[q] = a; }
+                }
+                __syncwarp();
+            }
+        }
+        if (lane < BM25_RANKS) rank[t * BM25_RANKS + lane] = (1 << lane) <= n ? f32_from_ordered_bits(key[(1 << lane) - 1]) : 0.f;
+        __syncwarp();
+    }
+}
+// terms with df > RK_TOP: one CTA per term.  Radix select (digits of 11, 11 and 10 bits from the top) of T = the RK_TOP-th
+// best key; then the < RK_TOP keys above T are collected and sorted, and ranks past them are T itself (ties)
+constexpr int RL_THREADS = 512;
+template <typename F>
+__device__ __forceinline__ void rank_for_each_key(const float* __restrict__ s, int64_t n, F f)
+{
+    const int64_t head = min(n, (int64_t)((16 - ((uintptr_t)s & 15)) & 15) / 4);      // scalars up to 16-byte alignment
+    if ((int64_t)threadIdx.x < head) f(f32_ordered_bits(s[threadIdx.x]));
+    const float4* s4 = reinterpret_cast<const float4*>(s + head);
+    const int64_t n4 = (n - head) / 4;
+    int64_t i = threadIdx.x;
+    for (; i + 3 * RL_THREADS < n4; i += 4 * RL_THREADS) {          // four independent 16-byte loads per thread in flight
+        float4 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = __ldg(s4 + i + u * RL_THREADS);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) { f(f32_ordered_bits(v[u].x)); f(f32_ordered_bits(v[u].y)); f(f32_ordered_bits(v[u].z)); f(f32_ordered_bits(v[u].w)); }
+    }
+    for (; i < n4; i += RL_THREADS) {
+        const float4 v = __ldg(s4 + i);
+        f(f32_ordered_bits(v.x)); f(f32_ordered_bits(v.y)); f(f32_ordered_bits(v.z)); f(f32_ordered_bits(v.w));
+    }
+    for (int64_t k = head + n4 * 4 + threadIdx.x; k < n; k += RL_THREADS) f(f32_ordered_bits(s[k]));
+}
+__global__ void __launch_bounds__(RL_THREADS)
+rank_large_kernel(const int64_t* __restrict__ off, const float* __restrict__ score, const uint32_t* __restrict__ terms,
+                  float* __restrict__ rank)
+{
+    typedef cub::BlockScan<uint32_t, RL_THREADS> Scan;
+    __shared__ typename Scan::TempStorage s_scan;
+    __shared__ uint32_t s_hist[2048];
+    __shared__ uint32_t s_top[RK_TOP];
+    __shared__ uint32_t s_prefix, s_need, s_cnt;
+    const int tid = threadIdx.x;
+    const uint32_t t = terms[blockIdx.x];
+    const int64_t b = off[t], df = off[t + 1] - b;
+    const float* s = score + b;
+    uint32_t prefix = 0, mask = 0, need = RK_TOP;                   // need: rank of T among the keys that match prefix
+    for (int pass = 0; pass < 3; ++pass) {
+        const int shift = pass == 0 ? 21 : (pass == 1 ? 10 : 0);
+        const uint32_t dmask = pass == 2 ? 0x3FFu : 0x7FFu;
+        for (int i = tid; i < 2048; i += RL_THREADS) s_hist[i] = 0;
+        __syncthreads();
+        rank_for_each_key(s, df, [&](uint32_t k) { if ((k & mask) == prefix) atomicAdd(&s_hist[(k >> shift) & dmask], 1u); });
+        __syncthreads();
+        // bins from the top: thread tid holds bins 2047 - 4 tid ... 2044 - 4 tid; the bin where the running count reaches
+        // `need` holds T
+        uint32_t c[4], sum = 0;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) { c[e] = s_hist[2047 - 4 * tid - e]; sum += c[e]; }
+        uint32_t above;
+        Scan(s_scan).ExclusiveSum(sum, above);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            if (above < need && above + c[e] >= need) { s_prefix = prefix | ((uint32_t)(2047 - 4 * tid - e) << shift); s_need = need - above; }
+            above += c[e];
+        }
+        __syncthreads();
+        prefix = s_prefix; need = s_need; mask |= dmask << shift;
+    }
+    // prefix == T; RK_TOP - need keys are above it
+    if (tid == 0) s_cnt = 0;
+    for (int i = tid; i < RK_TOP; i += RL_THREADS) s_top[i] = 0;
+    __syncthreads();
+    rank_for_each_key(s, df, [&](uint32_t k) { if (k > prefix) s_top[atomicAdd(&s_cnt, 1u)] = k; });
+    __syncthreads();
+    for (int k = 2; k <= RK_TOP; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int p = tid; p < RK_TOP / 2; p += RL_THREADS) {
+                const int i = ((p & ~(j - 1)) << 1) | (p & (j - 1)), q = i | j;
+                const uint32_t x = s_top[i], y = s_top[q];
+                if ((x < y) == ((i & k) == 0)) { s_top[i] = y; s_top[q] = x; }
+            }
+            __syncthreads();
+        }
+    }
+    const uint32_t n_above = RK_TOP - need;
+    if (tid < BM25_RANKS) rank[(int64_t)t * BM25_RANKS + tid] = f32_from_ordered_bits((1u << tid) <= n_above ? s_top[(1 << tid) - 1] : prefix);
+}
 // device scratch of the index build: everything allocated through it is freed on scope exit (also when a CUDA call
 // throws half-way), except what keep() hands over to the Postings
 struct DevScratch {
@@ -283,9 +395,18 @@ void build_postings(const uint32_t* term_ids, const uint16_t* term_tf, const uin
 
     uint32_t* post_doc = sc.alloc<uint32_t>((size_t)(nnz_live > 0 ? nnz_live : 1));
     float* post_score = sc.alloc<float>((size_t)(nnz_live > 0 ? nnz_live : 1));
+    float* rank_score = sc.alloc<float>((size_t)vocab * BM25_RANKS);
+    KRAG_CUDA(cudaMemsetAsync(rank_score, 0, sizeof(float) * (size_t)vocab * BM25_RANKS, st));
 
     if (nnz > 0 && nnz_live > 0) {
         prepare_tile_index(off, vocab, n_docs_rows, out, st);
+        // terms too long for a warp sort (df > RK_TOP), ascending: the ones of a term range are a contiguous run
+        std::vector<uint32_t> h_big;
+        for (int64_t t = 0; t < vocab; ++t)
+            if (h_off[(size_t)t + 1] - h_off[(size_t)t] > RK_TOP) h_big.push_back((uint32_t)t);
+        uint32_t* big = sc.alloc<uint32_t>(h_big.size());
+        if (!h_big.empty())
+            KRAG_CUDA(cudaMemcpyAsync(big, h_big.data(), sizeof(uint32_t) * h_big.size(), cudaMemcpyHostToDevice, st));
         // term ranges [t_lo, t_hi) of at most `cap` postings each (a single term longer than that is a range of its own).  The
         // sort buffers are sized for the widest range; if they do not fit after all (fragmentation, another context on the
         // device), the ranges are halved until they do
@@ -352,6 +473,17 @@ void build_postings(const uint32_t* term_ids, const uint16_t* term_tf, const uin
             count_launch();
             score_postings_kernel<<<148 * 8, 256, 0, st>>>(k_out, v_out, doc_len, idf, avgdl, m, post_doc + p_base, post_score + p_base);
             count_launch();
+            const int64_t small_grid = std::min<int64_t>((t_hi - t_lo + RS_WARPS - 1) / RS_WARPS, 148 * 16);
+            rank_small_kernel<<<(unsigned)small_grid, RS_WARPS * 32, 0, st>>>(off, post_score, t_lo, t_hi, rank_score);
+            KRAG_CUDA(cudaGetLastError());
+            count_launch();
+            const size_t b0 = std::lower_bound(h_big.begin(), h_big.end(), (uint32_t)t_lo) - h_big.begin();
+            const size_t b1 = std::lower_bound(h_big.begin(), h_big.end(), (uint32_t)t_hi) - h_big.begin();
+            if (b1 > b0) {
+                rank_large_kernel<<<(unsigned)(b1 - b0), RL_THREADS, 0, st>>>(off, post_score, big + b0, rank_score);
+                KRAG_CUDA(cudaGetLastError());
+                count_launch();
+            }
             if (out.n_slots > 0) {
                 tile_index_kernel<<<148 * 8, 256, 0, st>>>(k_out, post_doc, off, out.tile_slot, p_base, m, out.n_tiles, out.tile_off);
                 KRAG_CUDA(cudaGetLastError());
@@ -372,8 +504,9 @@ void build_postings(const uint32_t* term_ids, const uint16_t* term_tf, const uin
     if (out.off) cudaFree(out.off);
     if (out.doc) cudaFree(out.doc);
     if (out.score) cudaFree(out.score);
-    sc.keep(off); sc.keep(post_doc); sc.keep(post_score);
-    out.off = off; out.doc = post_doc; out.score = post_score; out.vocab = vocab; out.nnz = nnz_live;
+    if (out.rank_score) cudaFree(out.rank_score);
+    sc.keep(off); sc.keep(post_doc); sc.keep(post_score); sc.keep(rank_score);
+    out.off = off; out.doc = post_doc; out.score = post_score; out.rank_score = rank_score; out.vocab = vocab; out.nnz = nnz_live;
 }
 
 // -------------------------------------------------------------------------- query time
@@ -641,9 +774,13 @@ bm25_tile_kernel(const int64_t* __restrict__ post_off, const uint32_t* __restric
 // once (atomicExch resets the accumulator) and, if it passes the query's admission threshold, appended to the query's
 // candidate list in global memory (one warp-aggregated atomic per round).  No per-item sort, no per-item list.
 //
-// Threshold: a first pass over every `stride`-th sub-tile (no threshold) fills the lists with a sample; the P-th best
-// sampled key is a VALID bound (P real documents are at least that good), so the main pass over all sub-tiles admits
-// ~stride * P documents per query instead of every touched one, and bm25_select_kernel takes the exact top-P of them.
+// Threshold: scores are positive and fp32 round-to-nearest addition is monotone, so a document's sum is >= the score of
+// any one query term it contains.  Term t has at least 2^i postings scoring >= rank_score[t][i] (the rank table, built at
+// commit), hence for 2^i >= P the largest such entry over the query's terms bounds the query's P-th best score from below
+// (bm25_rank_threshold_kernel).  The pass over all sub-tiles admits only documents at or above it, and bm25_select_kernel
+// takes the exact top-P of them.  The table counts the documents that were alive at commit: when the bitmap of the call
+// admits fewer (a delete since, a pushdown filter), a first pass over every `stride`-th sub-tile (no threshold) fills the
+// lists with a sample instead, and its P-th best key is the bound (P real documents are at least that good).
 // A list that overflows (adversarial score layouts) raises the query's flag and the legacy kernel recomputes that query.
 //
 // Term -> posting range lookups: one u32 row of sub-tile boundaries per query term.  Frequent terms (> BM25_RARE_MAX
@@ -691,6 +828,23 @@ bm25_resolve_kernel(const uint32_t* __restrict__ q_terms, int n_terms, const int
         row[sidx] = (uint32_t)lo;
     }
     if (tid == 0) { q_row[i] = row; q_base[i] = b; q_slot[i] = -1; q_rare_len[i] = df; }
+}
+
+// per query: thr_q = the weakest key whose score is the largest rank-table entry of rank 2^lg >= P over its terms (every
+// tie at that score is admitted), or KEY_PAD (admit everything) when that is 0: out-of-vocabulary terms and terms with
+// fewer than 2^lg postings contribute nothing
+__global__ void bm25_rank_threshold_kernel(const uint32_t* __restrict__ q_terms, const int32_t* __restrict__ q_term_offsets,
+                                           int batch, const float* __restrict__ rank_score, int64_t vocab, int lg,
+                                           unsigned long long* __restrict__ thr_q)
+{
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= batch) return;
+    float s = 0.f;
+    for (int i = q_term_offsets[q]; i < q_term_offsets[q + 1]; ++i) {
+        const uint32_t t = q_terms[i];
+        if ((int64_t)t < vocab) s = fmaxf(s, rank_score[(int64_t)t * BM25_RANKS + lg]);
+    }
+    thr_q[q] = s > 0.f ? (make_key_desc(s, 0u) | 0xFFFFFFFFull) : KEY_PAD;
 }
 
 struct BwCtx {
@@ -1026,10 +1180,11 @@ static int bw_capq(int P)
     return c;
 }
 // which query kernel serves a shard: KRAG_BM25_KERNEL = auto (default) | warp | legacy; KRAG_BM25_LEGACY=1 == legacy.
-// auto: the warp kernel's fixed passes (resolve, sample pass, two selects) cost ~0.5 ms per batch whatever the shard size,
-// the first-generation kernel has almost none but ~1.5x the per-posting cost: the curves cross near 3M rows per shard
-// (measured: 10M rows 2.2 vs 3.1 ms, 1.25M rows 0.75 vs 0.50 ms per 256-query batch).
-constexpr int64_t BW_AUTO_MIN_ROWS = 3000000;
+// auto: with the rank-table threshold the warp kernel's fixed passes are a resolve, the threshold and one select; measured
+// per 256-query batch of the bench's queries (scripts/k3_cutover.py, B200 at 1000 W) warp vs first generation: 0.17 vs
+// 0.085 ms at 40k rows, 0.128 vs 0.110 at 80k, 0.128 vs 0.169 at 160k, 0.15 vs 0.24 at 320k, 0.27 vs 0.54 at 1.25M, 0.73 vs
+// 1.67 at 5M: the curves cross between 80k and 160k rows
+constexpr int64_t BW_AUTO_MIN_ROWS = 160000;
 static bool bw_legacy(int64_t n_rows)
 {
     if (env_int("KRAG_BM25_LEGACY", 0) != 0) return true;
@@ -1072,7 +1227,7 @@ size_t bm25_resolve_bytes(int64_t n_rows, int n_terms_total)
     return n * (8 + 8 + 4 + 4) + n * (size_t)(n_sub + 1) * 4 + 64;
 }
 
-void launch_bm25(const DeviceInfo& di, const Postings& post, int64_t n_rows, const uint32_t* alive,
+void launch_bm25(const DeviceInfo& di, const Postings& post, int64_t n_rows, const uint32_t* alive, bool alive_is_committed,
                  const uint32_t* q_terms, const int32_t* q_term_offsets, int n_terms_total, void* resolve_ws, int batch, int P,
                  OrdMap ord_base, uint64_t* part, uint64_t* keys_out, cudaStream_t st)
 {
@@ -1121,9 +1276,20 @@ void launch_bm25(const DeviceInfo& di, const Postings& post, int64_t n_rows, con
             KRAG_CUDA(cudaGetLastError());
             count_launch();
         };
-        if (!complete) {
-            // sample every stride-th sub-tile: the main pass then admits ~stride * P documents per query.  Small strides cost a
-            // larger sample pass (1 / stride of the main pass) but tighten the threshold: fewer candidate pushes, shorter final select
+        if (!complete && alive_is_committed) {
+            // the rank table was built over exactly the documents `alive` admits: its bound holds, no sample pass
+            int lg = 0;
+            while ((1 << lg) < P) ++lg;
+            bm25_rank_threshold_kernel<<<(batch + 127) / 128, 128, 0, st>>>(q_terms, q_term_offsets, batch, post.rank_score, post.vocab,
+                                                                         lg, thr_q);
+            KRAG_CUDA(cudaGetLastError());
+            count_launch();
+            pass(1, thr_q, counters);
+            need_safety_net = true;
+        } else if (!complete) {
+            // deletes since the commit or a pushdown filter: documents the rank table counted may be excluded, so its bound
+            // may not hold.  Sample every stride-th sub-tile instead: the main pass then admits ~stride * P documents per
+            // query.  Small strides cost a larger sample pass (1 / stride of the main pass) but tighten the threshold
             int stride = L.capq / (4 * P);
             if (stride > 64) stride = 64;
             if (stride < 1) stride = 1;

@@ -97,8 +97,12 @@ struct Postings {
     int32_t* tile_slot = nullptr;   // [vocab]  slot of a frequent term, -1 for the others
     uint32_t* tile_off = nullptr;   // [n_slots][n_tiles + 1]
     int64_t n_slots = 0, n_tiles = 0;   // n_tiles = number of BM25_SUB_DOCS ranges
+    // rank table: rank_score[t][i] = the 2^i-th best posting score of term t (the stored fp32 value), 0 when df(t) < 2^i.
+    // Any query containing t has at least 2^i documents scoring >= that value: K3's admission threshold without a sample pass
+    float* rank_score = nullptr;    // [vocab][BM25_RANKS]
 };
 constexpr int BM25_RARE_MAX = 2048;
+constexpr int BM25_RANKS = 11;      // ranks 1, 2, 4, ..., 1024 = KRAG_MAX_POOL
 void launch_df_histogram(const uint32_t* term_ids, const uint32_t* entry_doc, const uint32_t* alive, int64_t nnz,
                          uint32_t* df, cudaStream_t st);
 void launch_expand_entry_doc(const int64_t* term_offsets, int64_t n_docs, uint32_t* entry_doc, cudaStream_t st);
@@ -108,7 +112,9 @@ void build_postings(const uint32_t* term_ids, const uint16_t* term_tf, const uin
                     double avgdl, int64_t n_docs_rows, Postings& out, cudaStream_t st);
 size_t bm25_part_elems(int64_t n_rows, int batch, int P);
 size_t bm25_resolve_bytes(int64_t n_rows, int n_terms_total);   // size of launch_bm25's resolve_ws
-void launch_bm25(const DeviceInfo& di, const Postings& post, int64_t n_rows, const uint32_t* alive,
+// alive_is_committed: `alive` admits exactly the documents the postings were built from (no delete since the commit, no
+// filter), so the rank table bounds every query's P-th best score
+void launch_bm25(const DeviceInfo& di, const Postings& post, int64_t n_rows, const uint32_t* alive, bool alive_is_committed,
                  const uint32_t* q_terms, const int32_t* q_term_offsets, int n_terms_total, void* resolve_ws, int batch, int P,
                  OrdMap ord_base, uint64_t* part, uint64_t* keys_out, cudaStream_t st);
 
